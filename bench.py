@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- PDHG iterations/s of the B200 PDLP engine on BASELINE.json's synthetic LPs.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload S3|S2|S5] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload S3|S2|S5] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is ONE PDHG iteration of the hot path (primal step, A x + dual step, A'y +
 step rule) on the stated LP; the timed region runs exactly K iterations INCLUDING the
@@ -206,6 +206,15 @@ def parity_block(lp, lp_path, ours, L, ref_run):
         return {"error": str(e)[:300], "ok": False}
 
 
+def dump_outputs(dirpath, res):
+    """What the timed solve returned to its caller -- the four HighsSolution vectors -- as DIR/<name>.npy in float64, so
+    that two builds can be compared output for output (the inputs are seeded).  The largest workloads (n = m = 1e6) come
+    to 32 MB in all."""
+    os.makedirs(dirpath, exist_ok=True)
+    for k in ("col_value", "col_dual", "row_value", "row_dual"):
+        np.save(os.path.join(dirpath, k + ".npy"), np.asarray(res[k], dtype=np.float64))
+
+
 def cpu_cores():
     try:
         return len(os.sched_getaffinity(0))
@@ -314,6 +323,8 @@ def run_hipdlp_arm(args, device):
         (ia, ta), (ib, tb) = runs
         cpu = {"value": (ib - ia) / max(tb - ta, 1e-9), "unit": "iter/s", "cores": 1, "kind": "reference",
                "host_cores_available": cpu_cores(), "sample": f"HiGHS CPU hipdlp, {ib - ia} steady-state steps (two-point fit)"}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r)
     print(json.dumps({
         "metric": "pdhg_iterations_per_sec", "value": value, "unit": "iter/s", "n_gpus": 1, "steps": K, "warmup": W,
         "ms_per_step": r["loop_device_ms"] / K, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
@@ -347,7 +358,11 @@ def main():
     ap.add_argument("--to-tolerance", type=float, default=0.0,
                     help="additionally solve the workload to this kkt_tolerance through the host-buffer call and report the "
                          "wall-clock time to solution (SURVEY.md 8(d)); single GPU / reference arm")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the solution vectors the last timed solve returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what this engine computed; it does not apply to --impl reference")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -573,6 +588,8 @@ def main():
     }
     if tts is not None:
         line["time_to_solution"] = tts
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)
     print(json.dumps(line))
 
 

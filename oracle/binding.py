@@ -221,6 +221,14 @@ def _parse_json_line(text: str) -> dict:
     return json.loads(line)
 
 
+def driver_env() -> dict:
+    """Environment for the ref_driver binaries: the drop-in ones load highs_b200/libb200pdlp.so of THIS tree.  Their run path
+    cannot be relied on for it -- $ORIGIN resolves symlinks, so a linked or copied oracle/_ref/ no longer sits next to the
+    engine -- and LD_LIBRARY_PATH is searched before a run path."""
+    eng = os.path.join(os.path.dirname(HERE), "highs_b200")
+    return dict(os.environ, LD_LIBRARY_PATH=os.pathsep.join(p for p in (eng, os.environ.get("LD_LIBRARY_PATH")) if p))
+
+
 def ref_available() -> bool:
     return os.path.exists(REF_DRIVER)
 
@@ -261,7 +269,7 @@ def run_reference(lp=None, mps=None, options=None, want_solution=False, warm=Non
                 for v in (cv, cd, rv, rd):
                     f.write(np.asarray(v, dtype="<f8").tobytes())
             cmd += ["--warm", wp]
-        out = subprocess.run(cmd, capture_output=True, text=True, timeout=timeout)
+        out = subprocess.run(cmd, capture_output=True, text=True, timeout=timeout, env=driver_env())
         if out.returncode != 0:
             raise RuntimeError(f"ref_driver failed: {out.stderr}")
         res = _parse_json_line(out.stdout)

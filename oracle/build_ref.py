@@ -119,9 +119,11 @@ def main():
     keep = [o for o, s_ in zip(objs, srcs) if not s_.endswith("pdlp/CupdlpWrapper.cpp")]
     nj.append("rule cxxshim\n  command = g++ -std=c++11 $cxxflags_shim -c $in -o $out")
     nj.append(f"build {shim_o}: cxxshim {shim_src}\n  cxxflags_shim = {common} -I{os.path.join(os.path.dirname(HERE), 'include')}")
-    nj.append("rule linkshim\n  command = g++ -shared -o $out $in -L$engdir -lb200pdlp '-Wl,-rpath,$engdir' -lpthread -lm -ldl")
+    # the engine is found relative to oracle/_ref/ (not by absolute path), so a tree copied elsewhere still runs; an oracle/_ref/
+    # reached through a symlink needs oracle.binding.driver_env() (LD_LIBRARY_PATH), since $ORIGIN resolves symlinks
+    nj.append("rule linkshim\n  command = g++ -shared -o $out $in -L$engdir -lb200pdlp '-Wl,-rpath,$$ORIGIN/../../highs_b200' -lpthread -lm -ldl")
     nj.append(f"build {lib2}: linkshim {' '.join(keep)} {shim_o}\n  engdir = {eng_dir}")
-    nj.append("rule exeshim\n  command = g++ -std=c++11 -O2 $cxxincs $in -o $out -L$libdir -lhighs_b200 -L$engdir -lb200pdlp '-Wl,-rpath,$$ORIGIN' '-Wl,-rpath,$engdir' -lpthread")
+    nj.append("rule exeshim\n  command = g++ -std=c++11 -O2 $cxxincs $in -o $out -L$libdir -lhighs_b200 -L$engdir -lb200pdlp '-Wl,-rpath,$$ORIGIN' '-Wl,-rpath,$$ORIGIN/../../highs_b200' -lpthread")
     nj.append(f"build {drv2}: exeshim {os.path.join(HERE, 'ref_driver.cpp')} | {lib2}\n"
               f"  cxxincs = {incs} -w\n  libdir = {OUT}\n  engdir = {eng_dir}")
     # --- the same with the HiPDLP wrapper replaced as well (solver=hipdlp -> the engine's Halpern mode); kept in a THIRD
@@ -133,7 +135,7 @@ def main():
     keep3 = [o for o, s_ in zip(objs, srcs) if not s_.endswith("pdlp/CupdlpWrapper.cpp") and not s_.endswith("pdlp/HiPdlpWrapper.cpp")]
     nj.append(f"build {shim2_o}: cxxshim {shim2_src}\n  cxxflags_shim = {common} -I{os.path.join(os.path.dirname(HERE), 'include')}")
     nj.append(f"build {lib3}: linkshim {' '.join(keep3)} {shim_o} {shim2_o}\n  engdir = {eng_dir}")
-    nj.append("rule exeshim3\n  command = g++ -std=c++11 -O2 $cxxincs $in -o $out -L$libdir -lhighs_b200_hipdlp -L$engdir -lb200pdlp '-Wl,-rpath,$$ORIGIN' '-Wl,-rpath,$engdir' -lpthread")
+    nj.append("rule exeshim3\n  command = g++ -std=c++11 -O2 $cxxincs $in -o $out -L$libdir -lhighs_b200_hipdlp -L$engdir -lb200pdlp '-Wl,-rpath,$$ORIGIN' '-Wl,-rpath,$$ORIGIN/../../highs_b200' -lpthread")
     nj.append(f"build {drv3}: exeshim3 {os.path.join(HERE, 'ref_driver.cpp')} | {lib3}\n"
               f"  cxxincs = {incs} -w\n  libdir = {OUT}\n  engdir = {eng_dir}")
     if "--shim" in sys.argv and os.path.exists(os.path.join(eng_dir, "libb200pdlp.so")):

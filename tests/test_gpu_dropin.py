@@ -5,6 +5,7 @@ HighsLpSolverObject, lpKktCheck, HighsInfo -- is the reference's unmodified code
 import numpy as np
 import pytest
 
+import recorded_reference
 from conftest import case_id, golden_lp, golden_solution, load_golden
 
 pytestmark = pytest.mark.gpu
@@ -50,7 +51,7 @@ def test_presolved_lp_through_the_shim(oracle, name):
         pytest.skip("instance fixture missing")
     lp = read_b2lp(path)
     opts = {"presolve": "choose", "pdlp_iteration_limit": 20000}
-    ref = oracle.run_reference(lp=lp, options=opts)
+    ref = recorded_reference.run_reference(lp, options=opts)
     got = oracle.run_reference(lp=lp, options=opts, driver=oracle.DROPIN_DRIVER)
     assert got["model_status_code"] == ref["model_status_code"], (got["model_status"], ref["model_status"])
     assert got["pdlp_iteration_count"] == ref["pdlp_iteration_count"]
@@ -67,7 +68,7 @@ def test_pdlp_cleanup_with_the_engine(oracle):
         pytest.skip("oracle/_ref/ref_driver_b200 not built")
     lp = read_b2lp(os.path.join(GOLDEN, "instances", "standata.b2lp"))
     opts = {"presolve": "choose", "kkt_tolerance": 1e-4}
-    ref = oracle.run_reference(lp=lp, options=opts, pdlp_cleanup=1e3, cleanup_tighten=0.1)
+    ref = recorded_reference.run_reference(lp, options=opts, pdlp_cleanup=1e3, cleanup_tighten=0.1)
     got = oracle.run_reference(lp=lp, options=opts, pdlp_cleanup=1e3, cleanup_tighten=0.1, driver=oracle.DROPIN_DRIVER)
     for k in ("cleanup_considered", "cleanup_attempted", "cleanup_iteration_limit", "cleanup_first_status_code",
               "cleanup_first_pdlp_iterations", "model_status_code", "pdlp_iteration_count"):
@@ -93,7 +94,7 @@ def test_highs_run_hipdlp_through_the_shim(oracle, name):
         pytest.skip("instance fixture missing")
     lp = read_b2lp(path)
     opts = {"solver": "hipdlp", "presolve": "off", "pdlp_iteration_limit": 8000}
-    ref = oracle.run_reference(lp=lp, options=opts)
+    ref = recorded_reference.run_reference(lp, options=opts)
     got = oracle.run_reference(lp=lp, options=opts, driver=drv)
     assert got["model_status_code"] == ref["model_status_code"], (got["model_status"], ref["model_status"])
     assert got["pdlp_iteration_count"] == ref["pdlp_iteration_count"]

@@ -5,6 +5,7 @@ import os
 import numpy as np
 import pytest
 
+import recorded_reference
 from conftest import GOLDEN, golden_lp, load_golden
 
 
@@ -72,26 +73,23 @@ def test_golden_fixture_inventory():
     assert (lp.num_col_, lp.num_row_, lp.a_matrix_.numNz()) == (8, 10, 30)     # check/Avgas, BASELINE config 1
 
 
-def test_goldens_reproduce_from_reference(oracle):
-    """re-run the unmodified reference on two committed cases: tests/golden/golden.json is what it prints"""
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref not built")
+def test_goldens_reproduce_from_reference():
+    """the unmodified reference's runs of two committed cases (recorded in tests/golden/reference_runs.json): tests/golden/golden.json
+    is what it prints"""
     for c in load_golden():
         if (c["name"], c["tag"]) in (("avgas", "default"), ("distillation", "kkt1e-4")):
-            ref = oracle.run_reference(lp=golden_lp(c), options=c["options"])
+            ref = recorded_reference.run_reference(golden_lp(c), options=c["options"])
             assert ref["pdlp_iteration_count"] == c["pdlp_iteration_count"]
             assert ref["objective_function_value"] == c["objective_function_value"]
             assert ref["model_status_code"] == c["model_status_code"]
 
 
-def test_reference_kkt_evaluator(oracle):
+def test_reference_kkt_evaluator():
     """ref_driver --kkt-of = the reference's lpKktCheck on a GIVEN solution: fed the golden solution it must return the
     golden HighsInfo (this is the yard-stick the GPU parity tests use for 'KKT residuals')"""
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref not built")
     from conftest import golden_solution
     c = [c for c in load_golden() if (c["name"], c["tag"]) == ("afiro", "default")][0]
-    kkt = oracle.reference_kkt(golden_lp(c), golden_solution(c), c["model_status_code"], c["options"])
+    kkt = recorded_reference.reference_kkt(golden_lp(c), golden_solution(c), c["model_status_code"], c["options"])
     for k in ("max_primal_infeasibility", "max_dual_infeasibility", "primal_dual_objective_error",
               "max_complementarity_violation", "objective_function_value"):
         assert kkt[k] == c[k], k

@@ -1,5 +1,6 @@
 """The post-solve KKT assessment (highs_b200/csrc/kkt_logic.hpp + kkt_check.cu) against the reference's own lpKktCheck
-(/root/reference/highs/lp_data/HighsSolution.cpp:1043-1327, run through oracle/_ref/ref_driver --kkt-of): the HOST twin here
+(highs/lp_data/HighsSolution.cpp:1043-1327, run through oracle/_ref/ref_driver --kkt-of and recorded in
+tests/golden/reference_runs.json): the HOST twin here
 (no GPU); the device version is compared with both in tests/test_gpu_kkt.py.  Solutions: the committed goldens (reference
 output), loose and converged oracle solutions on instances with every row / bound type, and perturbed solutions so that
 every counter is exercised."""
@@ -8,6 +9,7 @@ import os
 import numpy as np
 import pytest
 
+import recorded_reference
 from conftest import GOLDEN, case_id, golden_lp, golden_solution, load_golden
 
 FLOAT_FIELDS = ("objective_function_value", "primal_dual_objective_error", "max_primal_infeasibility", "sum_primal_infeasibilities",
@@ -34,14 +36,12 @@ CASES = [c for c in load_golden() if c["model_status_code"] in (7, 14, 15) and g
 
 
 @pytest.mark.parametrize("case", CASES, ids=case_id)
-def test_host_twin_matches_reference_on_goldens(engine_lib, oracle, case):
+def test_host_twin_matches_reference_on_goldens(engine_lib, case):
     from highs_b200 import engine
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref/ref_driver not built")
     lp, sol = golden_lp(case), golden_solution(case)
     tol = case["options"].get("kkt_tolerance", 0.0)
     status_in = 7 if case["model_status_code"] in (7, 15) else case["model_status_code"]
-    ref = oracle.reference_kkt(lp, sol, model_status_code=status_in, options=case["options"])
+    ref = recorded_reference.reference_kkt(lp, sol, model_status_code=status_in, options=case["options"])
     ours = engine.kkt_check(lp, sol, kkt_tolerance=tol, model_status=status_in, on_device=False)
     compare(ours, ref)
 
@@ -51,8 +51,6 @@ def test_host_twin_matches_reference_on_goldens(engine_lib, oracle, case):
 def test_host_twin_matches_reference_on_instances(engine_lib, oracle, name, tol):
     from highs_b200 import engine
     from highs_b200.lp import read_b2lp
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref/ref_driver not built")
     path = os.path.join(GOLDEN, "instances", name + ".b2lp")
     if not os.path.exists(path):
         pytest.skip("instance fixture missing")
@@ -60,7 +58,7 @@ def test_host_twin_matches_reference_on_instances(engine_lib, oracle, name, tol)
     sol = oracle.solve(lp, tol_primal=tol, tol_dual=tol, tol_gap=tol, iter_limit=30000)
     for status_in, kt in ((7, tol), (15, tol), (7, 0.0)):
         opts = {"kkt_tolerance": kt} if kt else {}
-        ref = oracle.reference_kkt(lp, sol, model_status_code=status_in, options=opts)
+        ref = recorded_reference.reference_kkt(lp, sol, model_status_code=status_in, options=opts)
         ours = engine.kkt_check(lp, sol, kkt_tolerance=kt, model_status=status_in, on_device=False)
         compare(ours, ref)
     # a damaged solution: bound violations, wrong-sign duals, inconsistent activities
@@ -69,7 +67,7 @@ def test_host_twin_matches_reference_on_instances(engine_lib, oracle, name, tol)
     bad["col_value"] += 1e-2 * rng.standard_normal(lp.num_col_)
     bad["row_dual"] += 1e-2 * rng.standard_normal(lp.num_row_)
     bad["col_dual"] += 1e-3 * rng.standard_normal(lp.num_col_)
-    ref = oracle.reference_kkt(lp, bad, model_status_code=7)
+    ref = recorded_reference.reference_kkt(lp, bad, model_status_code=7)
     ours = engine.kkt_check(lp, bad, model_status=7, on_device=False)
     compare(ours, ref)
     assert ours["model_status"] == 15 and ours["num_primal_infeasibilities"] > 0

@@ -5,6 +5,7 @@ check/CMakeLists.txt:321-335) and full HighsSolution vectors.  The oracle must r
 import numpy as np
 import pytest
 
+import recorded_reference
 from conftest import (case_id, golden_lp, golden_solution, load_golden, options_to_params,
                       term_to_model_status)
 
@@ -51,9 +52,8 @@ def test_reference_goldens_of_its_own_tests():
 
 
 def test_oracle_vs_live_reference(oracle):
-    """fresh random LPs (equality, ranged, free rows, bounded columns, maximise) against oracle/_ref"""
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref not built")
+    """fresh random LPs (equality, ranged, free rows, bounded columns, maximise) against oracle/_ref (its runs recorded in
+    tests/golden/reference_runs.json)"""
     from highs_b200.lp import HighsLp, HighsSparseMatrix
     import scipy.sparse as sp
     rng = np.random.default_rng(42)
@@ -70,11 +70,11 @@ def test_oracle_vs_live_reference(oracle):
         lp = HighsLp(n, m, rng.standard_normal(n) + (1.0 if trial % 2 == 0 else 0.0), lo, up, rl, ru,
                      HighsSparseMatrix(n, m, A.indptr, A.indices, A.data), -1 if trial == 3 else 1, 0.5)
         opts = {"kkt_tolerance": 1e-4, "pdlp_iteration_limit": 20000}
-        ref = oracle.run_reference(lp=lp, options=opts, want_solution=True)
+        ref = recorded_reference.run_reference(lp, options=opts, want_solution=True)
         res = oracle.solve(lp, tol_primal=1e-4, tol_dual=1e-4, tol_gap=1e-4, iter_limit=20000)
         assert res["iters"] == ref["pdlp_iteration_count"]
         for k in ("col_value", "col_dual", "row_value", "row_dual"):
-            assert np.array_equal(res[k], ref[k]), (trial, k)
+            assert recorded_reference.digest(res[k]) == ref[k], (trial, k)
 
 
 @pytest.mark.parametrize("name", ["avgas", "afiro", "adlittle", "sctest", "chip", "boxed_row", "restart_lp"])

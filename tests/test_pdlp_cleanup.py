@@ -3,8 +3,8 @@
 highs_b200/csrc/highs_pdlp_cleanup.hpp restates -- through HiGHS's public API -- the clean-up flow the reference has compiled
 out (/root/reference/highs/lp_data/Highs.cpp:1940-1982, `consider_pdlp_cleanup = false`; decision rule
 Highs::tryPdlpCleanup, highs/lp_data/HighsInterface.cpp:4210-4272).  The helper is solver-agnostic, so its logic is checked
-HERE on the CPU against the unmodified reference library (oracle/_ref/ref_driver --pdlp-cleanup); tests/test_gpu_dropin.py
-repeats the flow with the B200 engine behind solver=pdlp."""
+HERE on the CPU against the unmodified reference library (oracle/_ref/ref_driver --pdlp-cleanup, its results recorded in
+tests/golden/reference_runs.json); tests/test_gpu_dropin.py repeats the flow with the B200 engine behind solver=pdlp."""
 import os
 
 import pytest
@@ -18,10 +18,9 @@ def _lp(name):
 
 
 @pytest.fixture(scope="module")
-def ref(oracle):
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref/ref_driver not built")
-    return oracle
+def ref():
+    import recorded_reference
+    return recorded_reference
 
 
 OPTS = {"presolve": "choose", "kkt_tolerance": 1e-4}

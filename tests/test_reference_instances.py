@@ -1,22 +1,18 @@
-"""Every LP the reference ships for its own tests (check/instances/*.mps, read by the unmodified reference through
-oracle/_ref/ref_driver) through the product's host prologue -- formulate + Ruiz/Pock-Chambolle scaling + transposition,
+"""Every LP the reference ships for its own tests (check/instances/*.mps as read by the unmodified reference, stored in
+tests/golden/instances/) through the product's host prologue -- formulate + Ruiz/Pock-Chambolle scaling + transposition,
 bit for bit against the oracle -- and through the device layouts of 1 and 3 ranks, evaluated on the host; and the
-oracle itself against the live reference on each of them (three option sets -- 400 iterations, 240 without restarts, to 1e-3 -- and a hot start from the reference's own 1e-3
-solution: iteration count and solution vectors, bit for bit).
-Needs /root/reference and oracle/_ref (development container only); about 20 s."""
+oracle itself against the reference's runs on each of them (three option sets -- 400 iterations, 240 without restarts, to 1e-3 -- and a hot start from the reference's own 1e-3
+solution: iteration count and solution vectors, bit for bit; recorded in tests/golden/reference_runs.json).
+About 20 s."""
 import json
 import os
 import subprocess
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/check/instances"), reason="reference tree not present")
-@pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "ref_driver")), reason="oracle/_ref not built")
-def test_reference_instances_through_host_prologue():
+def test_reference_instances_through_host_prologue(engine_lib):
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "sweep_reference_instances.py")], capture_output=True,
                        text=True, timeout=900, cwd=ROOT)
     lines = [ln for ln in r.stdout.splitlines() if ln.startswith("{")]

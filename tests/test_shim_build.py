@@ -28,9 +28,10 @@ def test_dropin_fails_loudly_without_gpu(engine_lib):
     from highs_b200 import engine
     if engine.device_count() > 0:
         pytest.skip("a GPU is visible")
-    from oracle.binding import _parse_json_line
+    from oracle.binding import _parse_json_line, driver_env
     out = subprocess.run([DRV, "--lp", os.path.join(GOLDEN, "avgas.b2lp"), "--opt", "solver=pdlp", "--opt", "presolve=off"],
-                         capture_output=True, text=True)
+                         capture_output=True, text=True, env=driver_env())
+    assert out.stdout.strip(), out.stderr[-2000:]
     res = _parse_json_line(out.stdout)
     assert res["run_status"] == -1 and res["model_status_code"] == 4          # HighsStatus::kError, kSolveError
     assert res["pdlp_iteration_count"] == -1

@@ -1,29 +1,22 @@
-"""Dev-container tool (reads /root/reference): every check/instances/*.mps of the reference through the host prologue
-(formulate + scale, bit for bit against the oracle) and the device layouts of 1 and 3 ranks (host evaluation against a
-plain sparse product), in reference order and length-sorted; and the oracle against the live reference (400 iterations,
-bit for bit) on each of them.
+"""Every LP the reference ships for its own tests (check/instances/*.mps as read by the reference, stored in
+tests/golden/instances/) through the host prologue (formulate + scale, bit for bit against the oracle) and the device
+layouts of 1 and 3 ranks (host evaluation against a plain sparse product), in reference order and length-sorted; and the
+oracle against the reference's runs (recorded in tests/golden/reference_runs.json; 400 iterations, bit for bit) on each of them.
 usage: python tools/sweep_reference_instances.py        last line: JSON {"ok": n, "bad": [[name, what], ...]}"""
-import glob, os, subprocess, sys, time
+import glob, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
+sys.path[:0] = [ROOT, os.path.join(ROOT, "tests")]
 import numpy as np
+import recorded_reference
 from highs_b200 import engine
 from highs_b200.lp import read_b2lp
 from oracle import binding as ob
 KEYS = ["cost", "lower", "upper", "rhs", "col_scale", "row_scale", "cbeg", "cidx", "cval", "row_new_idx", "row_type", "rbeg", "ridx", "rval"]
-drv = os.path.join(ROOT, "oracle", "_ref", "ref_driver")
-tmp = __import__("tempfile").mkdtemp(prefix="b200inst_")
+VECS = recorded_reference.VECTORS
 bad = []; n_ok = 0; n_pinned = 0; n_hot = 0
-for mps in sorted(glob.glob("/root/reference/check/instances/*.mps")):
-    name = os.path.basename(mps)[:-4]
-    out = f"{tmp}/{name}.b2lp"
-    try:
-        r = subprocess.run([drv, "--mps", mps, "--dump-lp", out, "--opt", "solver=pdlp", "--opt", "pdlp_iteration_limit=1", "--opt", "presolve=off"], capture_output=True, text=True, timeout=120)
-    except subprocess.TimeoutExpired:
-        print(name, "dump timeout"); continue
-    if not os.path.exists(out):
-        print(name, "no dump", r.stderr[-200:]); continue
-    lp = read_b2lp(out)
+for path in sorted(glob.glob(os.path.join(ROOT, "tests", "golden", "instances", "*.b2lp"))):
+    name = os.path.basename(path)[:-5]
+    lp = read_b2lp(path)
     if lp.num_row_ == 0 or lp.a_matrix_.numNz() == 0:
         print(name, "skipped (no rows / nnz)"); continue
     try:
@@ -47,17 +40,18 @@ for mps in sorted(glob.glob("/root/reference/check/instances/*.mps")):
             for opts, prm in (({"pdlp_iteration_limit": 400}, dict(iter_limit=400)),
                               ({"pdlp_iteration_limit": 240, "pdlp_cupdlpc_restart_method": 0}, dict(iter_limit=240, restart=0)),
                               ({"pdlp_iteration_limit": 1200, "kkt_tolerance": 1e-3}, dict(iter_limit=1200, tol_primal=1e-3, tol_dual=1e-3, tol_gap=1e-3))):
-                ref = ob.run_reference(lp=lp, options=opts, want_solution=True)
+                ref = recorded_reference.run_reference(lp, options=opts, want_solution=True, keep=("pdlp_iteration_count",) + VECS)
                 o = ob.solve(lp, **prm)
-                if ref["pdlp_iteration_count"] != o["iters"] or not all(np.array_equal(ref[k], o[k]) for k in ("col_value", "col_dual", "row_value", "row_dual")):
+                if ref["pdlp_iteration_count"] != o["iters"] or not all(recorded_reference.digest(o[k]) == ref[k] for k in VECS):
                     diffs.append(f"oracle vs reference {opts}: {ref['pdlp_iteration_count']} / {o['iters']} iterations")
-            # hot start (PDHG_PreSolve, cupdlp_solver.c:1217-1279): restart both from the reference's own 1e-3 solution
+            # hot start (PDHG_PreSolve, cupdlp_solver.c:1217-1279): restart both from the reference's own 1e-3 solution,
+            # which the last option set above has just found bit-equal to the oracle's
             # (Highs::setSolution recomputes the row activities of a user solution in quad precision before the wrapper sees
             #  them -- Highs.cpp:2519-2530, calculateRowValuesQuad, HighsLpUtils.cpp:3011-3047 -- and ranged rows start
             #  their slack from them, so the oracle is given the exactly rounded A x as well)
             if lp.a_matrix_.numNz() <= 20000:
                 from fractions import Fraction
-                w = ob.run_reference(lp=lp, options={"pdlp_iteration_limit": 1200, "kkt_tolerance": 1e-3}, want_solution=True)
+                w = o
                 accq = [Fraction(0)] * lp.num_row_
                 Am = lp.a_matrix_
                 for jc in range(lp.num_col_):
@@ -65,10 +59,10 @@ for mps in sorted(glob.glob("/root/reference/check/instances/*.mps")):
                     for pe in range(Am.start_[jc], Am.start_[jc + 1]):
                         accq[Am.index_[pe]] += xj * Fraction(float(Am.value_[pe]))
                 rvq = np.array([float(a_) for a_ in accq])
-                ref = ob.run_reference(lp=lp, options={"pdlp_iteration_limit": 200}, want_solution=True,
-                                       warm=(w["col_value"], w["col_dual"], w["row_value"], w["row_dual"]))
+                ref = recorded_reference.run_reference(lp, options={"pdlp_iteration_limit": 200}, want_solution=True,
+                                                       warm=tuple(w[k] for k in VECS), keep=("pdlp_iteration_count",) + VECS)
                 o = ob.solve(lp, iter_limit=200, warm=(w["col_value"], rvq, w["row_dual"]))
-                if ref["pdlp_iteration_count"] != o["iters"] or not all(np.array_equal(ref[k], o[k]) for k in ("col_value", "col_dual", "row_value", "row_dual")):
+                if ref["pdlp_iteration_count"] != o["iters"] or not all(recorded_reference.digest(o[k]) == ref[k] for k in VECS):
                     diffs.append(f"oracle vs reference, hot start: {ref['pdlp_iteration_count']} / {o['iters']} iterations")
                 n_hot += 1
             n_pinned += 1
